@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference          # the reference's CPU algorithm on the host cores
+    python bench.py --steps 2 --warmup 1 --dump-outputs out/   # + what the last timed step computed, as .npy
 
 A "step" is one pass of the hot path (exhaustive matching [+ two-view verification]) over every
 image pair of the synthetic scene.  Prints ONE JSON line (rank 0).
@@ -56,7 +57,14 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--pair-batch", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0's pairs, a seeded sample) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 class ClockSampler:
@@ -190,6 +198,47 @@ def pair_list(pb, cfg):
     return np.ascontiguousarray(np.concatenate(pb.exhaustive_pair_blocks(n, 50)))
 
 
+DUMP_BYTES = 64 * 10 ** 6    # everything --dump-outputs writes, .npy headers included
+DUMP_SUMMARY_PAIRS = 32768
+
+
+def dump_outputs(out_dir, res, pairs, feats, verify):
+    """--dump-outputs: what the caller of match_pairs received, one float .npy per array under out_dir.
+
+    The pairs are a seeded sample that depends on the pair count alone, never on the results, so that two builds
+    dump the same pairs.  For up to DUMP_SUMMARY_PAIRS of them, in pair-list order: `pairs` (image indices),
+    `num_matches` and, with verification, `config`, `num_inliers`, `E`, `F`, `H`, `cam2_from_cam1` (3 x 4) and
+    `tri_angle`.  For as many of those pairs as fit DUMP_BYTES even when every pair had `feats` matches (the most
+    one image can have), flagged by `has_lists`: their `matches` and `inlier_matches` concatenated in the same order
+    (`num_matches` / `num_inliers` of the flagged pairs split them)."""
+    order = np.random.default_rng(0).permutation(len(pairs))
+    summary = np.sort(order[:DUMP_SUMMARY_PAIRS])
+    ks = summary.tolist()
+    out = {"pairs": pairs[summary].astype(np.float64),
+           "num_matches": np.array([len(res.matches(k)) for k in ks], np.float64)}
+    if verify:
+        geoms = [res.two_view_geometry(k) for k in ks]
+        out["config"] = np.array([int(g.config) for g in geoms], np.float64)
+        out["num_inliers"] = np.array([len(g.inlier_matches) for g in geoms], np.float64)
+        for m in ("E", "F", "H"):
+            out[m] = np.stack([getattr(g, m) for g in geoms]).astype(np.float64)
+        out["cam2_from_cam1"] = np.stack([g.cam2_from_cam1.matrix() for g in geoms]).astype(np.float64)
+        out["tri_angle"] = np.array([g.tri_angle for g in geoms], np.float64)
+    fixed = sum(a.nbytes for a in out.values()) + len(summary) * 8 + (1 << 16)   # + has_lists, headers
+    per_pair = feats * 2 * 4 * (2 if verify else 1)                                # <= feats rows x 2, float32
+    listed = np.isin(summary, order[:max(0, (DUMP_BYTES - fixed) // per_pair)])
+    out["has_lists"] = listed.astype(np.float64)
+    pos = np.flatnonzero(listed)
+    out["matches"] = np.concatenate([res.matches(ks[i]) for i in pos] + [np.zeros((0, 2))]).astype(np.float32)
+    if verify:
+        out["inlier_matches"] = np.concatenate([geoms[i].inlier_matches for i in pos]
+                                               + [np.zeros((0, 2))]).astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    return sum(a.nbytes for a in out.values())
+
+
 def reference_arm(args, cfg, rank):
     """--impl reference: the reference's CPU algorithm (oracle port; the reference itself cannot be built here,
     DESIGN.md section 0) on the host cores, bounded sample of the same workload per step."""
@@ -291,9 +340,10 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def one_step(host=None):
+    def one_step(host=None, keep=False):
         """One pass of the hot path: shard -> whole set resident on this GPU (copy + ONE all-gather) -> match
-        (+ verify) this rank's pairs.  `host`: (desc, kpts) pinned host arrays of the local shard (e2e leg)."""
+        (+ verify) this rank's pairs.  `host`: (desc, kpts) pinned host arrays of the local shard (e2e leg).
+        `keep`: hand the result object back as out["res"] instead of freeing it."""
         w0 = time.perf_counter()
         if host is None:
             ctx.set_images_sharded(nfeat, first, count, d_desc.data_ptr(), d_kpts.data_ptr() if verify else None, cams,
@@ -312,7 +362,10 @@ def main():
             _ = res.matches(len(my_pairs) - 1)
             if verify:
                 _ = res.two_view_geometry(len(my_pairs) - 1)
-        res.free()
+        if keep:
+            out["res"] = res
+        else:
+            res.free()
         out["wall_ms"] = dict(upload=(w1 - w0) * 1e3, match_pairs=(w2 - w1) * 1e3, read_and_free=(time.perf_counter() - w2) * 1e3)
         return out
 
@@ -328,8 +381,8 @@ def main():
     t_wall0 = time.perf_counter()
     acc = dict(dev_ms=0.0, k1_ms=0.0, k1_n=0, ver_ms=0.0, ag_ms=0.0, up_ms=0.0)
     last = None
-    for _ in range(args.steps):
-        last = one_step()
+    for i in range(args.steps):
+        last = one_step(keep=bool(args.dump_outputs) and i == args.steps - 1)
         for k in acc:
             acc[k] += last[k]
     barrier()
@@ -339,6 +392,11 @@ def main():
     clk = clocks.stop() if rank == 0 else None
     st_end = ctx.stats()
     launches = st_end["kernel_launches"]
+    if args.dump_outputs:
+        if rank == 0:
+            nbytes = dump_outputs(args.dump_outputs, last["res"], my_pairs, K, verify)
+            log(f"outputs of the last timed step: {nbytes / 1e6:.1f} MB in {args.dump_outputs}")
+        last["res"].free()
 
     t = torch.tensor([acc["dev_ms"], wall_ms, acc["k1_ms"], acc["ag_ms"]], dtype=torch.float64, device=dev)
     cnt = torch.tensor([float(len(my_pairs)), float(launches), float(last["n_ver"]), float(last["matches"])],

@@ -32,6 +32,13 @@ def test_reference_arm_prints_one_contract_line():
     assert d["e2e"] == {"value": d["value"], "unit": "pairs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_rejects_zero_steps_and_dumping_the_reference_arm():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True,
+                             timeout=60, cwd=ROOT)
+        assert out.returncode == 2 and "error" in out.stderr and out.stdout == "", extra
+
+
 def test_reference_arm_is_silent_on_other_ranks():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     assert _run("--gpus", "2", env=env) == []
